@@ -16,6 +16,8 @@ mode R = MCP reframe + JSON side-band) per GPU, every stream complete in the bat
 
 Multi-GPU (torchrun, one rank per GPU): connections shard by hash(conn_id) % N, no collective on the data path.
 `--impl reference` times the reference's CPU path (the oracle port: the reference is Go and cannot be built here).
+`--dump-outputs DIR` writes what the last timed step computed as .npy files (dump_outputs): the inputs depend on the
+arguments alone, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -250,19 +252,98 @@ def bind_to_gpu_numa_node(torch, local_rank):
         return None
 
 
+def per_segment(res):
+    """(frames, frame bytes, records) each segment of a batch result delivers: its inline run plus the runs linked from it."""
+    cs = np.concatenate([[0], np.cumsum(res.frames["len"].astype(np.int64))])
+    ff, frames = res.segs["frame_first"].astype(np.int64), res.segs["frame_count"].astype(np.int64)
+    nbytes, recs = cs[ff + frames] - cs[ff], res.segs["rec_count"].astype(np.int64)
+    owner, cur = np.arange(len(res.segs)), res.segs["next"].astype(np.int64)
+    while True:
+        live = cur != 0xFFFFFFFF
+        owner, cur = owner[live], cur[live]
+        if not cur.size:
+            return frames, nbytes, recs
+        run = res.runs[cur]
+        a, b = run["frame_first"].astype(np.int64), run["frame_count"].astype(np.int64)
+        np.add.at(frames, owner, b)
+        np.add.at(nbytes, owner, cs[a + b] - cs[a])
+        np.add.at(recs, owner, run["rec_count"].astype(np.int64))
+        cur = run["next"].astype(np.int64)
+
+
 def delivered(res):
     """(frames, frame bytes) a batch result delivers: the inline run of every segment plus the runs linked from it."""
-    cs = np.concatenate([[0], np.cumsum(res.frames["len"].astype(np.int64))])
-    ff, fc = res.segs["frame_first"].astype(np.int64), res.segs["frame_count"].astype(np.int64)
-    frames, nbytes = int(fc.sum()), int((cs[ff + fc] - cs[ff]).sum())
-    cur = res.segs["next"].astype(np.int64)
-    cur = cur[cur != 0xFFFFFFFF]
-    while cur.size:
-        a, b = res.runs["frame_first"][cur].astype(np.int64), res.runs["frame_count"][cur].astype(np.int64)
-        frames += int(b.sum()); nbytes += int((cs[a + b] - cs[a]).sum())
-        cur = res.runs["next"][cur].astype(np.int64)
-        cur = cur[cur != 0xFFFFFFFF]
-    return frames, nbytes
+    frames, nbytes, _ = per_segment(res)
+    return int(frames.sum()), int(nbytes.sum())
+
+
+DUMP_BYTES = 64_000_000    # --dump-outputs writes at most this much
+DUMP_SEED = 0xD0           # seeds the order in which connections are sampled
+CONN_COLS = ("conn", "carry_len", "flags", "frames", "frame_bytes", "records")
+SAMPLE_COLS = ("conn", "frames", "records")
+REC_COLS = ("conn", "frame", "flags", "payload_len", "n_choices", "prompt_tokens", "completion_tokens", "total_tokens",
+            "content_len", "tool_calls")
+TC_COLS = ("record", "index", "has_id", "has_type", "has_function", "id_len", "type_len", "name_len", "args_len")
+
+
+def dump_outputs(res, out_dir):
+    """Writes what a caller receives from one batch result as <name>.npy under out_dir (at most DUMP_BYTES in all):
+      connections   one row per connection (CONN_COLS): its sse_seg_result and what it delivered
+      sample        the connections shown in full below, in a seeded order, as many as fit (SAMPLE_COLS)
+      frame_len, frame_bytes          their delivered frames in stream order, and the bytes of those frames
+      records, content_bytes          their delivered records (REC_COLS; frame = ordinal among the connection's frames,
+                                      -1 if not emitted; usage -1 when absent) and the content each carries
+      tool_calls, tool_call_bytes     the tool calls of those records (TC_COLS; record = row in records) and their id, type,
+                                      name and arguments
+    Arena offsets and table indices are resolved to what they point at, and the flag that says which arena a content
+    span lives in is cleared: the kernels place frames and records in whatever order their atomic allocations run, so
+    positions change from run to run while what a caller reads through them does not. A connections table larger than a
+    quarter of the budget keeps the first connections of the seeded order (sorted by id).
+    Returns the number of connections written in full."""
+    from inference_gateway_b200 import _abi as A
+    from tests.util import rec_to_dict
+    frames, nbytes, recs = per_segment(res)
+    n = len(res.segs)
+    order = np.random.default_rng(DUMP_SEED).permutation(n)
+    rows = np.sort(order[:min(n, DUMP_BYTES // 4 // (8 * len(CONN_COLS)))])
+    out = {"connections": np.stack([rows, res.segs["carry_len"][rows], res.segs["flags"][rows], frames[rows], nbytes[rows],
+                                    recs[rows]], axis=1).astype(np.float64)}
+    budget = DUMP_BYTES - 4096 - out["connections"].nbytes          # 4096: the .npy headers
+    sample, flen, fbytes, rec_rows, content, tc_rows, tc_bytes = [], [], [], [], [], [], []
+    for c in map(int, order):
+        fidx = [k for ff, fc, _, _ in res.seg_runs(c) for k in range(ff, ff + fc)]
+        fb = [res.at(int(res.frames[k]["off"]), int(res.frames[k]["len"])) for k in fidx]
+        ordinal = {k: j for j, k in enumerate(fidx)}
+        rr, cb, tr, tb = [], [], [], []
+        for ri in res.seg_recs(c):
+            d = rec_to_dict(res, ri)
+            tcs = d.get("tcs", [])
+            for t in tcs:
+                parts = [t["id"] or b"", t["type"] or b"", t["name"], t["args"]]
+                tr.append([len(rec_rows) + len(rr), t["index"], t["id"] is not None, t["type"] is not None, t["function"]]
+                          + [len(p) for p in parts])
+                tb.extend(parts)
+            cb.append(d.get("content", b""))
+            rr.append([c, ordinal.get(d["frame"], -1), d["flags"] & ~A.F_CONTENT_TEXT, d["payload_len"], d.get("n_choices", 0),
+                       *(d.get("usage") or (-1, -1, -1)), len(cb[-1]), len(tcs)])
+        cost = (4 * sum(map(len, fb + cb + tb)) + 8 * (len(SAMPLE_COLS) + len(fb) + len(REC_COLS) * len(rr)
+                                                       + len(TC_COLS) * len(tr)))
+        if cost > budget:
+            break
+        budget -= cost
+        sample.append([c, len(fb), len(rr)])
+        flen += map(len, fb); fbytes += fb; rec_rows += rr; content += cb; tc_rows += tr; tc_bytes += tb
+    out["sample"] = np.array(sample, dtype=np.float64).reshape(-1, len(SAMPLE_COLS))
+    out["frame_len"] = np.array(flen, dtype=np.float64)
+    out["frame_bytes"] = np.frombuffer(b"".join(fbytes), dtype=np.uint8).astype(np.float32)
+    out["records"] = np.array(rec_rows, dtype=np.float64).reshape(-1, len(REC_COLS))
+    out["content_bytes"] = np.frombuffer(b"".join(content), dtype=np.uint8).astype(np.float32)
+    out["tool_calls"] = np.array(tc_rows, dtype=np.float64).reshape(-1, len(TC_COLS))
+    out["tool_call_bytes"] = np.frombuffer(b"".join(tc_bytes), dtype=np.uint8).astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+    return len(sample)
 
 
 def main():
@@ -281,7 +362,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the rank to its GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs); "
+                         "under torchrun each rank writes to DIR/rank<r>")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.streams is None:
         args.streams = {"C2": 4096, "C3": 16384, "C4": 65536}[args.workload]
@@ -378,6 +466,10 @@ def main():
     sync_all()
     launches = eng.launch_count() - launches0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        out_dir = args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}")
+        n_full = dump_outputs(eng.download(slots[(args.steps - 1) % N_ROT][0], stream), out_dir)
+        log(f"[bench] outputs of the last timed step -> {out_dir} ({n_full} of {n_segs} connections in full)")
 
     # ---- the same streams in k seeded TCP pieces: a step is k launches, tails go through the carry slots
     segmented = None
@@ -473,7 +565,7 @@ def main():
 
         e2e_steps(depth)
         sync_all()
-        k_e2e = max(4, min(args.steps, 12))
+        k_e2e = args.steps
         t0 = time.perf_counter()
         fr = e2e_steps(k_e2e)
         torch.cuda.synchronize()
